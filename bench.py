@@ -43,6 +43,8 @@ LOCAL_BATCH = 32
 SEQ = 2048
 DDP_GLOBAL_BATCH = 256
 MODEL_NAMES = {"mpt-125m": "MPT-125M", "mpt-1b": "MPT-1B", "mpt-3b": "MPT-3B", "mpt-7b": "MPT-7B"}
+DUMP_PARAMS = 1 << 22       # --dump-outputs: at most this many fp32 parameters (16 MiB), a seeded sample of larger models
+DUMP_MAX_BYTES = 64 << 20
 
 
 def reference_arm() -> None:
@@ -211,6 +213,60 @@ class Env:
         return time.perf_counter() - t0, out
 
 
+# ------------------------------------------------------------------------------------------------------------------ outputs
+def param_sample(flat):
+    """A flat parameter vector as float32 on the host: whole up to ``DUMP_PARAMS`` elements, else the elements at ``DUMP_PARAMS``
+    positions drawn with a fixed seed (sorted, repeats dropped), so the same model size always yields the same positions."""
+    import numpy as np
+    import torch
+
+    flat = flat.detach().reshape(-1)
+    if flat.numel() > DUMP_PARAMS:
+        idx = np.unique(np.random.default_rng(0).integers(0, flat.numel(), DUMP_PARAMS))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    return flat.float().cpu().numpy()
+
+
+def fed_outputs(rt, results: list) -> dict:
+    """What a caller of one round receives: the new global model and every client's fit result, clients in id order.
+    ``num_examples`` is local steps x local batch; the cross-entropy is the mean over the client's local steps."""
+    import numpy as np
+
+    failed = [r for r in results if r.status.code != 0]
+    if failed:
+        raise SystemExit(f"bench round had failed clients: {failed[0].status.message}")
+    res = sorted(results, key=lambda r: int(r.cid))
+    n_layers = len(rt.model_layout.names)
+    return {"global_params": param_sample(rt.round_backend.global_params()),
+            "client_num_examples": np.array([r.num_examples for r in res], dtype=np.float64),
+            "client_cross_entropy": np.array([r.metrics["LanguageCrossEntropy"] for r in res], dtype=np.float64),
+            "client_pseudo_gradient_l2_norm": np.array([r.metrics["client/l2_norm_pseudo_gradient"] for r in res], dtype=np.float64),
+            "client_layer_pseudo_gradient_l2_norm": np.array(
+                [[r.metrics[f"client/layer/{i}/l2_norm_of_pseudo_gradient"] for i in range(n_layers)] for r in res], dtype=np.float64)}
+
+
+def ddp_outputs(tr, K: int) -> dict:
+    """What a caller of ``Trainer.fit`` receives: the trained parameters (this rank's, when they are sharded) and the loss of each
+    of the K steps of the call."""
+    import numpy as np
+
+    loss = [v for _, v in tr.loggers[0].data["loss/train/total"][-K:]]
+    return {"params": param_sample(tr.state.flat.params), "train_loss": np.array(loss, dtype=np.float64)}
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    import numpy as np
+
+    nbytes = sum(a.nbytes for a in arrays.values())
+    if nbytes > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {nbytes} bytes exceed the {DUMP_MAX_BYTES} byte budget")
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(d / f"{name}.npy", a)
+
+
 def run_fed(env: Env, args, impl: str, K: int, W: int) -> dict:
     """Configs #2 / #4 / #5: one federated round of K local steps per client + the round exchange."""
     torch = env.torch
@@ -257,8 +313,9 @@ def run_fed(env: Env, args, impl: str, K: int, W: int) -> dict:
     failed = [r for r in res if r.status.code != 0]
     if failed:
         raise SystemExit(f"bench round had failed clients: {failed[0].status.message}")
-    e2e_s, _ = env.walled(lambda: one_round(3))
+    e2e_s, res = env.walled(lambda: one_round(3))
     clk.stop()
+    outputs = fed_outputs(rt, res) if args.dump_outputs and impl == args.impl else None
     # the round exchange alone (aggregate + server optimizer + broadcast) on a freshly filled accumulator: device time of the
     # transport's launch, and wall clock of the whole public call (adds the host-side status agreement of the control plane)
     def fill() -> None:
@@ -283,7 +340,7 @@ def run_fed(env: Env, args, impl: str, K: int, W: int) -> dict:
                flops_per_token=float(mcfg.flops_per_token(SEQ)), optimizer=str(rt.cfg["llm_config"]["optimizer"]["name"]),
                comm_stack=rt.round_backend.name, microbatch=int(getattr(rt.trainer, "_auto_mb", None) or rt.trainer.microbatch),
                clients_per_node=n_clients // rt.n_nodes, gpus_per_client=gpc, n_clients=n_clients,
-               h2d=(n_clients // rt.n_nodes) * (LOCAL_BATCH // gpc) * SEQ * 8, d2h=(n_clients // rt.n_nodes) * 2 * 8)
+               h2d=(n_clients // rt.n_nodes) * (LOCAL_BATCH // gpc) * SEQ * 8, d2h=(n_clients // rt.n_nodes) * 2 * 8, outputs=outputs)
     rt.close()
     return out
 
@@ -315,6 +372,7 @@ def run_ddp(env: Env, args, impl: str, K: int, W: int) -> dict:
     launches = ops.launch_count() if impl == "ours" else 0
     e2e_s, _ = env.walled(lambda: tr.fit(duration=f"{K}ba"))
     clk.stop()
+    outputs = ddp_outputs(tr, K) if args.dump_outputs and impl == args.impl else None
     # the gradient all-reduce alone on the live bucket
     ar_ms = 0.0
     # (fully sharded: reduced per block inside the backward; fused ZeRO-1 step: the reduction is part of the step kernel)
@@ -335,7 +393,7 @@ def run_ddp(env: Env, args, impl: str, K: int, W: int) -> dict:
                clocks=clk.summary(), tokens=K * DDP_GLOBAL_BATCH * SEQ, flops_per_token=float(tr.model_cfg.flops_per_token(SEQ)),
                optimizer="decoupled_adamw", comm_stack=type(tr.grad_comm).__name__ if tr.grad_comm is not None else "none",
                microbatch=int(getattr(tr, "_auto_mb", None) or tr.microbatch), clients_per_node=1, gpus_per_client=env.world, n_clients=1,
-               h2d=per_gpu * SEQ * 8, d2h=2 * 8)
+               h2d=per_gpu * SEQ * 8, d2h=2 * 8, outputs=outputs)
     free_b, total_b = torch.cuda.mem_get_info(env.dev)
     out["gpu_mem_used_gb"] = round((total_b - free_b) / 2**30, 1)     # whole device, arena planes included (after the run)
     out["torch_peak_alloc_gb"] = round(torch.cuda.max_memory_allocated(env.dev) / 2**30, 1)
@@ -364,7 +422,13 @@ def main() -> None:
     ap.add_argument("--global-batch", type=int, default=0, help="ddp mode: sequences per optimizer step (default 256, BASELINE config #3)")
     ap.add_argument("--torch-arm", default="auto", choices=["auto", "on", "off"],
                     help="also measure the reference-equivalent stock-PyTorch arm in this invocation (auto = yes for mpt-125m)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps write what the timed path computed in its last step (fed: the new global model and the "
+                         "clients' fit results; ddp: the parameters and the step losses) as DIR/<name>.npy, float32 / float64, at most "
+                         "64 MiB; parameters of models above 4 Mi of them are a fixed, seeded sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.global_batch:
         global DDP_GLOBAL_BATCH
         DDP_GLOBAL_BATCH = int(args.global_batch)
@@ -377,6 +441,8 @@ def main() -> None:
     t_ours = time.time()
     r = run(env, args, args.impl, K, W)
     t_ours = time.time() - t_ours
+    if args.dump_outputs and env.rank == 0:
+        dump_outputs(args.dump_outputs, r["outputs"])
 
     def emit(torch_arm) -> None:
         if env.rank == 0:

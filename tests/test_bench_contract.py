@@ -36,15 +36,49 @@ def test_no_silent_cpu_fallback_and_launch_mismatch_is_reported():
         assert out.returncode != 0 and "CUDA" in (out.stderr + out.stdout) and not out.stdout.strip().startswith("{")
 
 
-def test_ddp_config_follows_the_sharding_switch():
-    """``--sharding``: plain DDP deletes ``fsdp_config`` (the launch scripts' choice), ``zero1`` / ``zero3`` keep it and name the scheme;
-    ``auto`` shards the 7B config fully and leaves the small ones replicated; ``--global-batch`` reaches the trainer config."""
-    import argparse
+def _bench_module():
     import importlib.util
 
     spec = importlib.util.spec_from_file_location("bench_mod", ROOT / "bench.py")
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_steps_below_one_are_rejected():
+    out = _run("--steps", "0")
+    assert out.returncode != 0 and "--steps" in out.stderr and not out.stdout.strip()
+
+
+def test_dump_outputs_writes_a_fixed_sample_within_budget(tmp_path, monkeypatch):
+    """``--dump-outputs``: small parameter vectors are written whole, large ones as the same seeded sample every time; only float32 /
+    float64 ``.npy`` files are written and a dump above the byte budget is refused."""
+    import numpy as np
+    import pytest
+
+    bench = _bench_module()
+    small = torch.arange(10, dtype=torch.float32)
+    assert np.array_equal(bench.param_sample(small), small.numpy())
+    monkeypatch.setattr(bench, "DUMP_PARAMS", 64)
+    big = torch.randn(10_000)
+    a, b = bench.param_sample(big), bench.param_sample(big.clone())
+    assert a.dtype == np.float32 and 0 < a.size <= 64 and np.array_equal(a, b)
+    assert np.isin(a, big.numpy()).all()
+    bench.dump_outputs(str(tmp_path / "out"), {"global_params": a, "loss": np.ones(3)})
+    assert np.array_equal(np.load(tmp_path / "out" / "global_params.npy"), a)
+    assert np.load(tmp_path / "out" / "loss.npy").dtype == np.float64
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 8)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "over"), {"loss": np.ones(3)})
+    assert not (tmp_path / "over").exists()
+
+
+def test_ddp_config_follows_the_sharding_switch():
+    """``--sharding``: plain DDP deletes ``fsdp_config`` (the launch scripts' choice), ``zero1`` / ``zero3`` keep it and name the scheme;
+    ``auto`` shards the 7B config fully and leaves the small ones replicated; ``--global-batch`` reaches the trainer config."""
+    import argparse
+
+    bench = _bench_module()
 
     def cfg(model, sharding, impl="ours"):
         a = argparse.Namespace(model=model, precision="amp_bf16", attention="b200", sharding=sharding)
