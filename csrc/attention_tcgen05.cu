@@ -29,6 +29,7 @@
 #include "attention_tcgen05.h"
 #include "gemm_tcgen05.h"
 #include "ptx.cuh"
+#include "rope.cuh"
 
 namespace pb {
 
@@ -1118,22 +1119,11 @@ __global__ void __launch_bounds__(256) rope_kernel(__nv_bfloat16* __restrict__ q
     const long long t = r / 2;
     const int pos = int(t % S);
     __nv_bfloat16* base = qkv + t * (3LL * H * dh) + (long long)which * H * dh + h * dh + g * 8;
-    const uint4 a = *reinterpret_cast<const uint4*>(base);
-    const uint4 b = *reinterpret_cast<const uint4*>(base + half);
-    const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, bw[4] = {b.x, b.y, b.z, b.w};
-    uint32_t oa[4], ob[4];
-    const float* c = cosT + (long long)pos * half + g * 8;
-    const float* sn = sinT + (long long)pos * half + g * 8;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const float2 x1 = unpack_bf16(aw[k]), x2 = unpack_bf16(bw[k]);
-      const float c0 = c[2 * k], c1 = c[2 * k + 1];
-      const float s0 = inverse ? -sn[2 * k] : sn[2 * k], s1 = inverse ? -sn[2 * k + 1] : sn[2 * k + 1];
-      oa[k] = pack_bf16(x1.x * c0 - x2.x * s0, x1.y * c1 - x2.y * s1);
-      ob[k] = pack_bf16(x2.x * c0 + x1.x * s0, x2.y * c1 + x1.y * s1);
-    }
-    *reinterpret_cast<uint4*>(base) = make_uint4(oa[0], oa[1], oa[2], oa[3]);
-    *reinterpret_cast<uint4*>(base + half) = make_uint4(ob[0], ob[1], ob[2], ob[3]);
+    uint4 a = *reinterpret_cast<const uint4*>(base);
+    uint4 b = *reinterpret_cast<const uint4*>(base + half);
+    rope_rotate8(a, b, cosT + (long long)pos * half + g * 8, sinT + (long long)pos * half + g * 8, inverse);
+    *reinterpret_cast<uint4*>(base) = a;
+    *reinterpret_cast<uint4*>(base + half) = b;
   }
 }
 }  // namespace

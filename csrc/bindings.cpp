@@ -6,6 +6,7 @@
 #include <pybind11/pybind11.h>
 #include <torch/extension.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <cstdlib>
@@ -14,6 +15,7 @@
 #include <vector>
 
 #include "comm.h"
+#include "decode.h"
 #include "fp8_ops.h"
 #include "fused_ops.h"
 #include "gemm_tcgen05.h"
@@ -404,6 +406,103 @@ void fused_optimizer(Tensor& p, const Tensor& g, Tensor& m, Tensor& v, c10::opti
   g_launches += 1;
 }
 
+// ---------------------------------------------------------------------------------- KV-cached decoding
+inline void check_i32(const Tensor& t, const char* name, int64_t n) {
+  check_cuda(t, name);
+  TORCH_CHECK(t.scalar_type() == at::kInt && t.is_contiguous() && t.numel() == n, name, " must be a contiguous int32 tensor of ", n,
+              " elements");
+}
+// embedding rows at explicit positions: out[t] = wte[ids[t]] (+ wpe[pos[t]])
+void embed_at(const Tensor& ids, const Tensor& pos, const Tensor& wte, const c10::optional<Tensor>& wpe, Tensor& out) {
+  check_cuda(ids, "ids");
+  TORCH_CHECK(ids.scalar_type() == at::kLong && ids.is_contiguous(), "ids must be contiguous int64");
+  check_i32(pos, "pos", ids.numel());
+  check_bf16(wte, "wte");
+  check_bf16(out, "out");
+  const int64_t d = wte.size(1);
+  TORCH_CHECK(out.is_contiguous() && out.numel() == ids.numel() * d, "out must be contiguous [T, d]");
+  if (wpe.has_value()) {
+    check_bf16(*wpe, "wpe");
+    TORCH_CHECK(wpe->dim() == 2 && wpe->size(1) == d, "wpe must be [max_pos, d]");
+  }
+  c10::cuda::CUDAGuard guard(ids.device());
+  pb::embed_fwd(ids.data_ptr<int64_t>(), wte.data_ptr(), opt_ptr(wpe), out.data_ptr(), ids.numel(), wpe.has_value() ? int(wpe->size(0)) : 1,
+                int(d), int(wte.size(0)), stream_of(ids), pos.data_ptr<int>());
+  g_launches += 1;
+}
+int64_t decode_attention_splits(int64_t BH, int64_t s_max) {
+  return pb::decode_attention_splits(int(BH), int(s_max), at::cuda::getCurrentDeviceProperties()->multiProcessorCount);
+}
+// q: [B, >= d] rows (row stride ldq, e.g. the q third of qkv [B, 3d]); kv: [B, S_max, 2d]; lengths int32 [B]; out [B, d]
+void decode_attention(const Tensor& q, const Tensor& kv, const Tensor& lengths, const c10::optional<Tensor>& alibi_slopes, double scale,
+                      int n_heads, int n_split, Tensor& out, c10::optional<Tensor> lse) {
+  check_bf16(q, "q");
+  check_bf16(kv, "kv");
+  check_bf16(out, "out");
+  TORCH_CHECK(kv.dim() == 3 && kv.is_contiguous(), "kv must be a contiguous [B, S_max, 2d] cache");
+  const int B = int(kv.size(0)), S = int(kv.size(1)), d = int(kv.size(2) / 2);
+  TORCH_CHECK(n_heads > 0 && d % n_heads == 0, "d must be a multiple of n_heads");
+  const int dh = d / n_heads;
+  TORCH_CHECK(dh == 64 || dh == 128, "decode_attention covers d_head 64 and 128");
+  TORCH_CHECK(q.dim() == 2 && q.size(0) == B && q.size(1) >= d && q.stride(1) == 1 && q.stride(0) % 8 == 0, "q must be [B, >= d] rows");
+  TORCH_CHECK(out.dim() == 2 && out.size(0) == B && out.size(1) == d && out.is_contiguous(), "out must be contiguous [B, d]");
+  check_i32(lengths, "lengths", B);
+  if (alibi_slopes.has_value()) {
+    check_f32(*alibi_slopes, "alibi_slopes");
+    TORCH_CHECK(alibi_slopes->numel() == n_heads && alibi_slopes->is_contiguous(), "alibi_slopes must have n_heads elements");
+  }
+  if (lse.has_value()) {
+    check_f32(*lse, "lse");
+    TORCH_CHECK(lse->is_contiguous() && lse->numel() == int64_t(B) * n_heads, "lse must be contiguous [B, H]");
+  }
+  c10::cuda::CUDAGuard guard(q.device());
+  const int max_split = (S + pb::DECODE_TILE_KEYS - 1) / pb::DECODE_TILE_KEYS;
+  if (n_split <= 0) n_split = pb::decode_attention_splits(B * n_heads, S, at::cuda::getCurrentDeviceProperties()->multiProcessorCount);
+  TORCH_CHECK(n_split <= std::max(max_split, 1), "n_split must be <= ceil(S_max / ", pb::DECODE_TILE_KEYS, ")");
+  Tensor scratch;
+  if (n_split > 1) scratch = torch::empty({int64_t(B) * n_heads * n_split * (dh + 2)}, q.options().dtype(at::kFloat));
+  g_launches += pb::decode_attention_launch(q.data_ptr(), q.stride(0), kv.data_ptr(), B, S, n_heads, dh, lengths.data_ptr<int>(),
+                                            alibi_slopes.has_value() ? alibi_slopes->data_ptr<float>() : nullptr, float(scale), n_split,
+                                            n_split > 1 ? scratch.data_ptr<float>() : nullptr, out.data_ptr(),
+                                            lse.has_value() ? lse->data_ptr<float>() : nullptr, stream_of(q));
+}
+// cache[b_idx[t], pos[t]] = k|v of qkv row t (after RoPE of q and k at pos[t] when cos / sin are given)
+void kv_write(Tensor& qkv, Tensor& cache, const Tensor& b_idx, const Tensor& pos, const c10::optional<Tensor>& cos_t,
+              const c10::optional<Tensor>& sin_t, int n_heads) {
+  check_bf16(qkv, "qkv");
+  check_bf16(cache, "cache");
+  TORCH_CHECK(qkv.dim() == 2 && qkv.is_contiguous(), "qkv must be contiguous [T, 3d]");
+  TORCH_CHECK(cache.dim() == 3 && cache.is_contiguous() && cache.size(2) * 3 == qkv.size(1) * 2, "cache must be contiguous [B, S_max, 2d]");
+  const int64_t T = qkv.size(0);
+  const int d = int(qkv.size(1) / 3);
+  TORCH_CHECK(n_heads > 0 && d % n_heads == 0, "d must be a multiple of n_heads");
+  const int dh = d / n_heads;
+  check_i32(b_idx, "b_idx", T);
+  check_i32(pos, "pos", T);
+  const bool rotate = cos_t.has_value();
+  TORCH_CHECK(rotate == sin_t.has_value(), "cos and sin go together");
+  if (rotate) {
+    check_f32(*cos_t, "cos");
+    check_f32(*sin_t, "sin");
+    TORCH_CHECK(cos_t->is_contiguous() && sin_t->is_contiguous() && cos_t->size(0) >= cache.size(1) && cos_t->size(1) == dh / 2 &&
+                    sin_t->sizes() == cos_t->sizes(), "cos/sin must be [>= S_max, dh/2]");
+  }
+  c10::cuda::CUDAGuard guard(qkv.device());
+  pb::kv_write_launch(qkv.data_ptr(), qkv.stride(0), cache.data_ptr(), int(cache.size(0)), int(cache.size(1)), b_idx.data_ptr<int>(),
+                      pos.data_ptr<int>(), rotate ? cos_t->data_ptr<float>() : nullptr, rotate ? sin_t->data_ptr<float>() : nullptr, T,
+                      n_heads, dh, rotate, stream_of(qkv));
+  g_launches += 1;
+}
+void argmax_rows(const Tensor& logits, Tensor& out) {
+  check_bf16(logits, "logits");
+  TORCH_CHECK(logits.dim() == 2 && logits.stride(1) == 1, "logits must be [R, V] with unit inner stride");
+  check_cuda(out, "out");
+  TORCH_CHECK(out.scalar_type() == at::kLong && out.is_contiguous() && out.numel() == logits.size(0), "out must be contiguous int64 [R]");
+  c10::cuda::CUDAGuard guard(logits.device());
+  pb::argmax_rows_launch(logits.data_ptr(), logits.stride(0), logits.size(0), int(logits.size(1)), out.data_ptr<int64_t>(), stream_of(logits));
+  g_launches += 1;
+}
+
 // ---------------------------------------------------------------------------------- symmetric arena (CUDA IPC)
 int64_t ipc_alloc(int64_t nbytes, int device) {
   c10::cuda::CUDAGuard guard(static_cast<c10::DeviceIndex>(device));
@@ -616,6 +715,13 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("axpby", &axpby);
   m.def("cast_bf16", &cast_bf16);
   m.def("fused_optimizer", &fused_optimizer);
+  m.def("embed_at", &embed_at);
+  m.def("decode_attention_splits", &decode_attention_splits);
+  m.def("decode_attention", &decode_attention, py::arg("q"), py::arg("kv"), py::arg("lengths"), py::arg("alibi_slopes"), py::arg("scale"),
+        py::arg("n_heads"), py::arg("n_split"), py::arg("out"), py::arg("lse") = py::none());
+  m.def("kv_write", &kv_write);
+  m.def("argmax_rows", &argmax_rows);
+  m.attr("DECODE_TILE_KEYS") = pb::DECODE_TILE_KEYS;
   m.def("ipc_alloc", &ipc_alloc);
   m.def("ipc_get_handle", &ipc_get_handle);
   m.def("ipc_open_handle", &ipc_open_handle);

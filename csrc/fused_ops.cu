@@ -43,15 +43,17 @@ __device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
 
 // ------------------------------------------------------------------ embedding
 // h[t,:] = wte[ids[t],:] + wpe[t % S,:]      (bf16 tables = compute shadow of the fp32 masters)
+// With `pos` (int32 [T], decoding: one row per sequence at its own position) the position is pos[t], clamped to [0, S).
 __global__ void embed_fwd_kernel(const int64_t* __restrict__ ids, const __nv_bfloat16* __restrict__ wte,
                                  const __nv_bfloat16* __restrict__ wpe, __nv_bfloat16* __restrict__ out, long long T,
-                                 int S, int d, int V) {
+                                 int S, int d, int V, const int* __restrict__ pos) {
   const int vec = d / 8;
   for (long long t = blockIdx.x; t < T; t += gridDim.x) {
     long long id = ids[t];
     id = id < 0 ? 0 : (id >= V ? V - 1 : id);
     const uint4* a = reinterpret_cast<const uint4*>(wte + id * d);
-    const uint4* b = wpe ? reinterpret_cast<const uint4*>(wpe + (long long)(t % S) * d) : nullptr;
+    const int p = pos ? min(max(pos[t], 0), S - 1) : int(t % S);
+    const uint4* b = wpe ? reinterpret_cast<const uint4*>(wpe + (long long)p * d) : nullptr;
     uint4* o = reinterpret_cast<uint4*>(out + t * d);
     for (int i = threadIdx.x; i < vec; i += blockDim.x) {
       float x[8], y[8];
@@ -665,9 +667,10 @@ inline int grid_for(long long work_items, int block, int max_blocks = 148 * 8) {
     if (e__ != cudaSuccess) throw std::runtime_error(std::string(name " launch: ") + cudaGetErrorString(e__)); \
   } while (0)
 
-void embed_fwd(const int64_t* ids, const void* wte, const void* wpe, void* out, long long T, int S, int d, int V, cudaStream_t st) {
+void embed_fwd(const int64_t* ids, const void* wte, const void* wpe, void* out, long long T, int S, int d, int V, cudaStream_t st,
+               const int* pos) {
   embed_fwd_kernel<<<grid_for(T, 1, 148 * 16), 128, 0, st>>>(ids, (const __nv_bfloat16*)wte, (const __nv_bfloat16*)wpe,
-                                                            (__nv_bfloat16*)out, T, S, d, V);
+                                                            (__nv_bfloat16*)out, T, S, d, V, pos);
   PB_CHECK_LAUNCH("embed_fwd");
 }
 void embed_bwd(const int64_t* ids, const void* dh, float* dwte, float* dwpe, long long T, int S, int d, int V, cudaStream_t st) {

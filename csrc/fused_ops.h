@@ -15,7 +15,9 @@ struct OptimHyper {
   float inv_sqrt_bc2;  // AdamW: 1 / sqrt(1 - beta2^t)
 };
 
-void embed_fwd(const int64_t* ids, const void* wte, const void* wpe, void* out, long long T, int S, int d, int V, cudaStream_t st);
+// pos: optional int32 [T] explicit positions (nullptr = t % S); S is then the number of rows of wpe
+void embed_fwd(const int64_t* ids, const void* wte, const void* wpe, void* out, long long T, int S, int d, int V, cudaStream_t st,
+               const int* pos = nullptr);
 void embed_bwd(const int64_t* ids, const void* dh, float* dwte, float* dwpe, long long T, int S, int d, int V, cudaStream_t st);
 void layernorm_fwd(const void* x, const float* gamma, const float* beta, void* y, float* mean, float* rstd, long long T, int d,
                    float eps, cudaStream_t st);

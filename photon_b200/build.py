@@ -19,7 +19,7 @@ CSRC = ROOT / "csrc"
 OBJ = ROOT / "build" / "obj"
 EXT_NAME = "_C"
 
-CU_SOURCES = ["gemm_tcgen05.cu", "gemm_mxfp8.cu", "attention_tcgen05.cu", "fused_ops.cu", "fp8_ops.cu", "comm.cu"]
+CU_SOURCES = ["gemm_tcgen05.cu", "gemm_mxfp8.cu", "attention_tcgen05.cu", "fused_ops.cu", "fp8_ops.cu", "comm.cu", "decode.cu"]
 CPP_SOURCES = ["bindings.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--use_fast_math", "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr"]

@@ -194,7 +194,7 @@ def build_icl_suite(cfg: Any, max_seq_len: int) -> Any:
 
     tok_cfg = dict((cfg["llm_config"].get("tokenizer") or {}))
     tokenizer = build_tokenizer(str(tok_cfg.get("name", "EleutherAI/gpt-neox-20b")))
-    return lambda logits_fn: run_icl_suite(logits_fn, tokenizer, cfg, max_seq_len)
+    return lambda logits_fn, generate_fn=None: run_icl_suite(logits_fn, tokenizer, cfg, max_seq_len, generate_fn=generate_fn)
 
 
 @dataclasses.dataclass

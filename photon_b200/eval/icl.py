@@ -9,10 +9,11 @@ self-contained implementation of the two task types that dominate those tables:
 * ``multiple_choice``     — pick the choice with the highest length-normalised log-likelihood;
   ``schema`` tasks are scored the same way with the context varying instead of the continuation.
 
-* ``generation_task_with_answers`` — greedy decoding (one ``logits_fn`` call per new token, no KV cache: this is an
-  evaluation utility, not a serving path) until ``max_new_tokens`` or an ``early_stopping_criteria`` string; exact match
-  against any of the ``answer`` / ``aliases`` after llm-foundry's normalisation (lower-case, punctuation and articles
-  stripped) unless ``do_normalization: false``; with a ``cot_delimiter`` only the text after it counts.
+* ``generation_task_with_answers`` — greedy decoding until ``max_new_tokens`` or an ``early_stopping_criteria`` string;
+  exact match against any of the ``answer`` / ``aliases`` after llm-foundry's normalisation (lower-case, punctuation and
+  articles stripped) unless ``do_normalization: false``; with a ``cot_delimiter`` only the text after it counts. With a
+  ``generate_fn`` (a backend's ``generate``: on the B200 engine, KV-cached decoding on its own kernels) the rows are
+  generated ``batch_size`` at a time; without one, row by row with one ``logits_fn`` call per new token.
 
 Datasets are jsonl files resolved against ``icl_tasks_config.root_dir`` (there is no network, so missing files yield
 ``skipped``).
@@ -53,11 +54,25 @@ def _rows(path: Path) -> list[dict[str, Any]]:
     return [json.loads(l) for l in path.read_text().splitlines() if l.strip()]
 
 
-class ICLEvaluator:
-    """``logits_fn(ids [B,S] LongTensor) -> [B,S,V]`` abstracts the model (torch backend or engine)."""
+GenerateFn = Callable[[list[list[int]], int, "int | None", "Callable[[int, list[int]], bool] | None"], list[list[int]]]
 
-    def __init__(self, logits_fn: Callable[[torch.Tensor], torch.Tensor], tokenizer: Any, max_seq_len: int, root_dir: str | None = None) -> None:
+
+def _cut_at_stop(text: str, stops: list[str]) -> str | None:
+    """``text`` up to the earliest stop string, or None when no stop string occurs."""
+    hit = [text.index(s) for s in stops if s and s in text]
+    return text[: min(hit)] if hit else None
+
+
+class ICLEvaluator:
+    """``logits_fn(ids [B,S] LongTensor) -> [B,S,V]`` abstracts the model (torch backend or engine).
+
+    ``generate_fn(prompts, max_new_tokens, eos_id, stop) -> new ids per prompt`` (optional): batched greedy decoding for the
+    generation tasks, ``stop(row, new_ids) -> bool`` ending a row; the backends' ``generate`` has this signature."""
+
+    def __init__(self, logits_fn: Callable[[torch.Tensor], torch.Tensor], tokenizer: Any, max_seq_len: int, root_dir: str | None = None,
+                 generate_fn: GenerateFn | None = None) -> None:
         self.logits_fn, self.tok, self.max_seq_len, self.root = logits_fn, tokenizer, int(max_seq_len), Path(root_dir or ".")
+        self.generate_fn = generate_fn
 
     def _enc(self, text: str) -> list[int]:
         if hasattr(self.tok, "encode") and not hasattr(self.tok, "__call__"):
@@ -95,11 +110,30 @@ class ICLEvaluator:
             if eos is not None and nxt == eos:
                 break
             ids.append(nxt), new.append(nxt)
-            text = self.tok.decode(new)
-            hit = [text.index(s) for s in stops if s and s in text]
-            if hit:
-                return text[: min(hit)]
+            cut = _cut_at_stop(self.tok.decode(new), stops)
+            if cut is not None:
+                return cut
         return self.tok.decode(new)
+
+    def _generate_batch(self, ctxs: list[list[int]], max_new_tokens: int, stops: list[str]) -> list[str]:
+        """:meth:`_generate` for many prompts in one ``generate_fn`` call: the same texts, stop strings checked on the decoded
+        text of each row after every token."""
+        stop = (lambda r, new: _cut_at_stop(self.tok.decode(new), stops) is not None) if any(stops) else None
+        outs = self.generate_fn(ctxs, max_new_tokens, getattr(self.tok, "eos_token_id", None), stop)
+        texts = [self.tok.decode(o) for o in outs]
+        return [t if (c := _cut_at_stop(t, stops)) is None else c for t in texts]
+
+    @staticmethod
+    def _score_generation(text: str, row: dict[str, Any], t: dict[str, Any]) -> int:
+        """1 when the generated ``text`` (after ``cot_delimiter``) matches the answer or an alias, else 0."""
+        if t["cot_delimiter"] and t["cot_delimiter"] in text:
+            text = text.split(t["cot_delimiter"])[-1]
+        golds = [str(row["answer"])] + [str(a) for a in row.get("aliases", [])]
+        norm = _normalize_answer if t["do_normalization"] else (lambda x: x.strip())
+        return int(any(norm(text).startswith(norm(g)) for g in golds if norm(g)))
+
+    def _generation_prompt(self, rows: list[dict[str, Any]], i: int, k: int, t: dict[str, Any]) -> list[int]:
+        return self._enc(self._fewshot_prefix(rows, i, k, t) + t["question_prelimiter"] + rows[i]["context"] + t["continuation_delimiter"].rstrip())
 
     def evaluate_task(self, task: dict[str, Any]) -> dict[str, float | str]:
         t = expand_task(task)
@@ -113,18 +147,20 @@ class ICLEvaluator:
             return {"status": "generation tasks need a tokenizer with decode()"}
         rows = _rows(path)
         out: dict[str, float | str] = {}
+        stops = list(t["early_stopping_criteria"] or [])
+        batched = kind == "generation_task_with_answers" and self.generate_fn is not None
         for k in t["num_fewshot"]:
             correct = 0
-            for i, r in enumerate(rows):
+            bs = max(1, int(t["batch_size"]))
+            for lo in range(0, len(rows), bs) if batched else ():
+                ctxs = [self._generation_prompt(rows, i, k, t) for i in range(lo, min(lo + bs, len(rows)))]
+                texts = self._generate_batch(ctxs, int(t["max_new_tokens"]), stops)
+                correct += sum(self._score_generation(text, rows[lo + j], t) for j, text in enumerate(texts))
+            for i, r in enumerate(rows if not batched else ()):
                 prefix = self._fewshot_prefix(rows, i, k, t)
                 if kind == "generation_task_with_answers":
-                    ctx = self._enc(prefix + t["question_prelimiter"] + r["context"] + t["continuation_delimiter"].rstrip())
-                    text = self._generate(ctx, int(t["max_new_tokens"]), list(t["early_stopping_criteria"] or []))
-                    if t["cot_delimiter"] and t["cot_delimiter"] in text:
-                        text = text.split(t["cot_delimiter"])[-1]
-                    golds = [str(r["answer"])] + [str(a) for a in r.get("aliases", [])]
-                    norm = _normalize_answer if t["do_normalization"] else (lambda x: x.strip())
-                    correct += int(any(norm(text).startswith(norm(g)) for g in golds if norm(g)))
+                    text = self._generate(self._generation_prompt(rows, i, k, t), int(t["max_new_tokens"]), stops)
+                    correct += self._score_generation(text, r, t)
                 elif kind == "language_modeling":
                     ctx = self._enc(prefix + t["question_prelimiter"] + r["context"] + t["continuation_delimiter"].rstrip())
                     _, em = self._continuation_stats(ctx, self._enc(" " + r["continuation"].lstrip()))
@@ -188,11 +224,13 @@ class EvalGauntlet:
         return out
 
 
-def run_icl_suite(logits_fn: Callable[[torch.Tensor], torch.Tensor], tokenizer: Any, cfg: Any, max_seq_len: int) -> dict[str, Any]:
-    """Evaluate every task of ``cfg.icl_tasks_config`` and fold through ``cfg.eval_gauntlet_config``."""
+def run_icl_suite(logits_fn: Callable[[torch.Tensor], torch.Tensor], tokenizer: Any, cfg: Any, max_seq_len: int,
+                  generate_fn: GenerateFn | None = None) -> dict[str, Any]:
+    """Evaluate every task of ``cfg.icl_tasks_config`` and fold through ``cfg.eval_gauntlet_config``; ``generate_fn``
+    batches the generation tasks (see :class:`ICLEvaluator`)."""
     icl = cfg.get("icl_tasks_config") or {}
     tasks = icl.get("icl_tasks") or []
-    ev = ICLEvaluator(logits_fn, tokenizer, max_seq_len, icl.get("root_dir"))
+    ev = ICLEvaluator(logits_fn, tokenizer, max_seq_len, icl.get("root_dir"), generate_fn=generate_fn)
     metrics: dict[str, Any] = {}
     for t in tasks:
         metrics.update({k: v for k, v in ev.evaluate_task(dict(t)).items() if not (k == "status")})

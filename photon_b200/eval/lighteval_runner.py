@@ -27,7 +27,7 @@ from typing import Any, Callable
 
 import torch
 
-from photon_b200.eval.icl import ICLEvaluator
+from photon_b200.eval.icl import GenerateFn, ICLEvaluator
 
 MULTIPLE_CHOICE = {"hellaswag", "arc", "piqa", "mmlu_pro", "commonsense_qa", "openbook_qa", "winogrande"}
 GENERATIVE = {"trivia_qa": {}, "gsm8k": {"cot_delimiter": "####", "max_new_tokens": 256, "early_stopping_criteria": ["\n\n"]},
@@ -60,8 +60,9 @@ def to_icl_task(entry: dict[str, Any]) -> dict[str, Any] | None:
 
 
 def run_task_list(tasks_file: str | Path, logits_fn: Callable[[torch.Tensor], torch.Tensor], tokenizer: Any, max_seq_len: int,
-                  data_root: str | Path) -> dict[str, Any]:
-    ev = ICLEvaluator(logits_fn, tokenizer, max_seq_len, str(data_root))
+                  data_root: str | Path, generate_fn: GenerateFn | None = None) -> dict[str, Any]:
+    """Score every entry of ``tasks_file``; ``generate_fn`` (a backend's ``generate``) batches the generative tasks."""
+    ev = ICLEvaluator(logits_fn, tokenizer, max_seq_len, str(data_root), generate_fn=generate_fn)
     results: dict[str, Any] = {}
     for entry in parse_task_list(tasks_file):
         key = f"{entry['suite']}|{entry['task']}|{entry['num_fewshot']}"
@@ -96,20 +97,33 @@ def main() -> None:
     cfg = compose([f"llm_config={a.model_config}"])
     mcfg = MPTConfig.from_model_cfg(dict(cfg["llm_config"]["model"]))
     dev = torch.device("cuda" if torch.cuda.is_available() else "cpu")
-    if dev.type == "cpu" and mcfg.attn_impl == "flash":
-        mcfg.attn_impl = "torch"
-    model = MPTForCausalLM(mcfg, device=dev, seed=17)
-    if a.checkpoint:
-        flat = FlatParams(model, device=dev, with_grad=False)
-        flat.load_ndarrays(load_model_parameters_from_file(a.checkpoint)[: len(flat.names)])
-    model.eval()
+    generate_fn = None
+    if dev.type == "cuda":
+        # the B200 engine: logits through its module view of the weights, generation KV-cached on its own kernels
+        from photon_b200.train.backend import build_backend
 
-    @torch.no_grad()
-    def logits_fn(ids: torch.Tensor) -> torch.Tensor:
-        with torch.autocast(dev.type, dtype=torch.bfloat16, enabled=dev.type == "cuda"):
+        backend = build_backend(mcfg, dev, "amp_bf16", seed=17)
+        if a.checkpoint:
+            backend.flat.load_ndarrays(load_model_parameters_from_file(a.checkpoint)[: len(backend.flat.names)])
+            backend.params_updated()
+        backend.train_mode(False)
+        logits_fn = backend.logits
+        if getattr(backend, "can_generate", False):
+            generate_fn = backend.generate
+    else:
+        if mcfg.attn_impl == "flash":
+            mcfg.attn_impl = "torch"
+        model = MPTForCausalLM(mcfg, device=dev, seed=17)
+        if a.checkpoint:
+            flat = FlatParams(model, device=dev, with_grad=False)
+            flat.load_ndarrays(load_model_parameters_from_file(a.checkpoint)[: len(flat.names)])
+        model.eval()
+
+        @torch.no_grad()
+        def logits_fn(ids: torch.Tensor) -> torch.Tensor:
             return model(ids.to(dev))
 
-    res = run_task_list(a.tasks, logits_fn, build_tokenizer(a.tokenizer), mcfg.max_seq_len, a.data_root)
+    res = run_task_list(a.tasks, logits_fn, build_tokenizer(a.tokenizer), mcfg.max_seq_len, a.data_root, generate_fn=generate_fn)
     text = json.dumps(res, indent=1)
     if a.out:
         Path(a.out).write_text(text)

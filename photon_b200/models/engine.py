@@ -27,7 +27,7 @@ backend and the two are directly comparable in tests.
 from __future__ import annotations
 
 import math
-from typing import Any
+from typing import Any, Callable
 
 import torch
 import torch.nn.functional as F
@@ -124,6 +124,7 @@ class B200Engine:
         self.launches_per_microbatch = 0
         self._ws: dict[tuple[int, int], dict[str, Any]] = {}
         self._stats = torch.zeros(4, dtype=torch.float64, device=self.device)
+        self._gen_decoder: Decoder | None = None    # kept between generate() calls of one evaluation
         self._bind()
         if self.fp8:
             self._init_fp8(int(kernels.get("fp8_amax_history_len", 16)), int(kernels.get("fp8_margin", 0)))
@@ -234,8 +235,10 @@ class B200Engine:
             self._fp8_calibrated = bool(sd.get("calibrated", True))
 
     # ---------------------------------------------------------------- workspace
-    def _workspace(self, b: int, S: int) -> dict[str, Any]:
-        key = (b, S)
+    def _workspace(self, b: int, S: int, fp8: bool | None = None) -> dict[str, Any]:
+        """``fp8=False`` on an amp_fp8 engine: bf16 block buffers (the decoder's prefill runs the bf16 GEMMs)."""
+        use8 = self.fp8 if fp8 is None else bool(fp8)
+        key = (b, S, use8)
         if key in self._ws:
             return self._ws[key]
         self._ws.clear()  # one live shape at a time (activations dominate memory)
@@ -249,7 +252,7 @@ class B200Engine:
             if self.activation_checkpointing and i > 0:
                 ws["layers"].append(ws["layers"][0])  # ONE set of block internals shared by all layers
                 continue
-            if self.fp8:   # the GEMM inputs exist only as E4M3 (1 byte): 7·T·d instead of 12·T·d bytes of saved activations
+            if use8:   # the GEMM inputs exist only as E4M3 (1 byte): 7·T·d instead of 12·T·d bytes of saved activations
                 u8 = lambda *s: torch.empty(*s, dtype=torch.uint8, device=dev)  # noqa: E731
                 ws["layers"].append({"ln1": u8(T, d), "m1": f32(T), "r1": f32(T), "qkv": bf(T, 3 * d), "attn": bf(T, d), "attn8": u8(T, d),
                                      "lse": f32(b, H, S), "hmid": bf(T, d), "ln2": u8(T, d), "m2": f32(T), "r2": f32(T),
@@ -267,7 +270,7 @@ class B200Engine:
         ws.update(lnf=bf(T, d), mf=f32(T), rf=f32(T), dlnf=bf(T, d), dh=bf(T, d), dhmid=bf(T, d), dln=bf(T, d),
                   dqkv=bf(T, 3 * d), dattn=bf(T, d), dz=bf(T, c.expansion_ratio * d), delta=f32(b, H, S),
                   logits=bf(min(self.lm_head_chunk, T), c.vocab_size))
-        if self.fp8:   # E5M2 copy of the gradient currently flowing backward (one buffer, viewed at the width in use)
+        if use8:   # E5M2 copy of the gradient currently flowing backward (one buffer, viewed at the width in use)
             ws["g8"] = torch.empty(T * max(c.expansion_ratio, 3) * d, dtype=torch.uint8, device=dev)
         self._ws[key] = ws
         return ws
@@ -313,10 +316,12 @@ class B200Engine:
         if self.rope is not None:
             ops.rope_(ws["dqkv"].view(b, S, 3 * c.d_model), self.rope[0], self.rope[1], c.n_heads, inverse=True)
 
-    def _block_fwd(self, i: int, ws: dict[str, Any], b: int, S: int) -> None:
-        """h[i] -> h[i+1]; the block internals land in ws["layers"][i] (also the recompute step under checkpointing)."""
+    def _block_fwd(self, i: int, ws: dict[str, Any], b: int, S: int, fp8: bool | None = None) -> None:
+        """h[i] -> h[i+1]; the block internals land in ws["layers"][i] (also the recompute step under checkpointing).
+        ``fp8=False`` runs the bf16 GEMMs on an amp_fp8 engine (decoder prefill)."""
         c, h, w, lw = self.cfg, ws["h"], self.layers[i], ws["layers"][i]
-        if self.fp8:
+        use8 = self.fp8 if fp8 is None else bool(fp8)
+        if use8:
             M, w8, R = self.fp8_meta, self.w8_views[i], self._role
             ops.layernorm_fwd_q8(h[i], w.g1, w.b1, lw["ln1"], lw["m1"], lw["r1"], c.norm_eps, M, R("x_ln1", i))
             ops.gemm_fp8(lw["ln1"], w8["wqkv"], lw["qkv"], M, R("x_ln1", i), R("wqkv", i), bias=w.bqkv)
@@ -335,7 +340,7 @@ class B200Engine:
         if self.rope is not None:
             ops.rope_(lw["qkv"].view(b, S, 3 * c.d_model), self.rope[0], self.rope[1], c.n_heads)
         self._attention_fwd(lw, b, S)
-        if self.fp8:
+        if use8:
             ops.colsum_quant(lw["attn"], None, lw["attn8"], ops.E4M3, M, R("x_attn", i))
             ops.gemm_fp8(lw["attn8"], w8["wo"], lw["hmid"], M, R("x_attn", i), R("wo", i), epi=ops.EPI_RESIDUAL, bias=w.bo, aux=h[i])
             ops.layernorm_fwd_q8(lw["hmid"], w.g2, w.b2, lw["ln2"], lw["m2"], lw["r2"], c.norm_eps, M, R("x_ln2", i))
@@ -541,12 +546,203 @@ class B200Engine:
         with torch.autocast("cuda", dtype=torch.bfloat16):
             return self.model(ids.to(self.device))
 
+    # --------------------------------------------------------------- generation
+    @property
+    def can_generate(self) -> bool:
+        """KV-cached decoding runs on this engine: unsharded weights, the tcgen05 attention path with d_head 64 / 128, and a
+        ``max_seq_len`` that is a multiple of the 128-row prefill tiles. Under amp_fp8 decoding reads the bf16 shadow with
+        the bf16 GEMMs (there is no fp8 decode path)."""
+        return (self.zero3 is None and self.attn_mode == "b200" and self.cfg.d_head in (64, 128)
+                and self.cfg.max_seq_len % 128 == 0)
+
+    def decoder(self, batch: int, max_len: int) -> "Decoder":
+        """A decoding session for ``batch`` rows of up to ``max_len`` tokens (prompt + generated) over this engine's weights."""
+        if not self.can_generate:
+            raise NotImplementedError("KV-cached decoding needs zero3=None, attention=b200, d_head 64/128 and max_seq_len % 128 == 0")
+        return Decoder(self, batch, max_len)
+
+    @torch.no_grad()
+    def generate(self, prompts: list[list[int]], max_new_tokens: int, eos_id: int | None = None,
+                 stop: Callable[[int, list[int]], bool] | None = None) -> list[list[int]]:
+        """Greedy continuation of every prompt, batched, with a KV cache; returns the new ids of each row.
+
+        Same semantics as per-row recompute (``ICLEvaluator._generate`` over :meth:`logits`): prompts are left-truncated to
+        ``max_seq_len``; a row ends at ``eos_id`` (not included), when ``stop(row, new_ids)`` returns True, or after
+        ``max_new_tokens``. A row whose context outgrows ``max_seq_len`` continues over its last ``max_seq_len`` ids,
+        recomputed through :meth:`logits` at each such step (its positions shift, so the cache no longer applies)."""
+        B, msl = len(prompts), self.cfg.max_seq_len
+        new: list[list[int]] = [[] for _ in range(B)]
+        if B == 0 or max_new_tokens <= 0:
+            return new
+        ctx = [list(p)[-msl:] for p in prompts]
+        need = min(msl, max(len(c) for c in ctx) + max_new_tokens)
+        dec = self._gen_decoder
+        if dec is None or dec.B != B or dec.S_max < need:
+            self._gen_decoder = None     # free the old cache first
+            dec = self._gen_decoder = self.decoder(B, need)
+        nxt = ops.argmax_rows(dec.prefill(ctx), out=dec.next_ids)
+        host = torch.empty(B, dtype=torch.int64, pin_memory=True)
+        done, windowed, wtok = [False] * B, [False] * B, [0] * B
+        for it in range(max_new_tokens):
+            host.copy_(nxt, non_blocking=True)
+            torch.cuda.current_stream(self.device).synchronize()
+            toks = host.tolist()
+            for r in range(B):
+                if done[r]:
+                    continue
+                t = wtok[r] if windowed[r] else toks[r]
+                if eos_id is not None and t == eos_id:
+                    done[r] = True
+                    continue
+                new[r].append(t)
+                ctx[r].append(t)
+                if stop is not None and stop(r, new[r]):
+                    done[r] = True
+            if all(done) or it == max_new_tokens - 1:
+                break
+            for r in range(B):
+                if not done[r] and len(ctx[r]) > msl:
+                    windowed[r] = True
+                    wtok[r] = int(self.logits(torch.tensor([ctx[r][-msl:]], device=self.device))[0, -1].float().argmax())
+            active = [not (done[r] or windowed[r]) for r in range(B)]
+            if any(active):
+                nxt = ops.argmax_rows(dec.step(nxt, active), out=dec.next_ids)
+        return new
+
     def train_mode(self, on: bool = True) -> None:
+        if on:
+            self._gen_decoder = None      # the KV cache does not outlive the evaluation
         if self.model is not None:
             self.model.train(on)
         elif on:
             self._eval_model = None       # the whole-model evaluation copy (full sharding) does not outlive the evaluation
 
     def close(self) -> None:
+        self._gen_decoder = None
         self._graphs.clear()
         self._ws.clear()
+
+
+class Decoder:
+    """KV-cached decoding session of a :class:`B200Engine`: the engine's bf16 weight shadow and fp32 small parameters, a
+    per-layer cache ``[B, S_max, 2d]`` (k | v, head-major like ``qkv``) and static step buffers.
+
+    :meth:`prefill` runs the engine's own block forward over the right-padded prompts and writes every layer's k | v into
+    the cache; :meth:`step` feeds one token per row through LN → QKV GEMM → (clip, qk-LN) → ``kv_write`` (RoPE at the row's
+    position) → ``decode_attention`` → out-projection + residual → LN → up + GELU → down + residual, then the final LN and
+    the LM head, all with ``M = B``. With ``kernels.cuda_graph`` the step is captured once and replayed: its shapes are
+    static and the per-row lengths are read on the device."""
+
+    def __init__(self, eng: B200Engine, batch: int, max_len: int) -> None:
+        c, dev = eng.cfg, eng.device
+        self.eng, self.B = eng, int(batch)
+        if self.B < 1:
+            raise ValueError("a decoder needs at least one row")
+        self.S_max = min(c.max_seq_len, -(-max(1, int(max_len)) // 128) * 128)
+        d, B = c.d_model, self.B
+        bf = lambda *s: torch.empty(*s, dtype=torch.bfloat16, device=dev)  # noqa: E731
+        f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)  # noqa: E731
+        self.cache = [bf(B, self.S_max, 2 * d) for _ in range(c.n_layers)]
+        self.lengths = [0] * B
+        self.meta = torch.zeros(2, B, dtype=torch.int32, device=dev)     # [0] = lengths, [1] = position of the step's token
+        self.b_idx = torch.arange(B, dtype=torch.int32, device=dev)
+        self.tokens = torch.zeros(B, dtype=torch.int64, device=dev)
+        self.next_ids = torch.zeros(B, dtype=torch.int64, device=dev)
+        self.h = [bf(B, d), bf(B, d)]
+        self.buf = {"ln": bf(B, d), "m": f32(B), "r": f32(B), "qkv": bf(B, 3 * d), "attn": bf(B, d), "hmid": bf(B, d),
+                    "z": bf(B, c.expansion_ratio * d), "u": bf(B, c.expansion_ratio * d)}
+        if c.qk_ln:
+            self.buf.update(qk_pre=bf(B, d), qk_tmp=bf(B, d))
+        self.logits = bf(B, c.vocab_size)
+        self.n_split = ops.decode_attention_splits(B * c.n_heads, self.S_max)
+        self._graph: Any = None
+
+    @torch.no_grad()
+    def prefill(self, prompts: list[list[int]]) -> torch.Tensor:
+        """Fill the cache with ``prompts`` (one per row, 1..S_max ids); returns the next-token logits ``[B, V]`` of every row."""
+        eng, c = self.eng, self.eng.cfg
+        if len(prompts) != self.B:
+            raise ValueError(f"prefill needs {self.B} prompts, got {len(prompts)}")
+        lens = [len(p) for p in prompts]
+        if min(lens) < 1 or max(lens) > self.S_max:
+            raise ValueError(f"prompt lengths must be within 1..{self.S_max}")
+        # right padding to the 128-row attention tiles: every pad key sits after every valid key, so causal attention over
+        # the valid positions is unchanged
+        S = -(-max(lens) // 128) * 128
+        ids = torch.zeros(self.B, S, dtype=torch.int64)
+        for r, p in enumerate(prompts):
+            ids[r, : len(p)] = torch.tensor(p, dtype=torch.int64)
+        ids = ids.to(eng.device)
+        ws = eng._workspace(self.B, S, fp8=False)
+        ops.embed_fwd(ids.reshape(-1), eng.wte16, eng.wpe16, ws["h"][0], S)
+        b_idx = self.b_idx.repeat_interleave(S)
+        pos = torch.arange(S, dtype=torch.int32, device=eng.device).repeat(self.B)
+        for i in range(c.n_layers):
+            eng._block_fwd(i, ws, self.B, S, fp8=False)
+            # right after the block: under activation checkpointing the next block overwrites the shared buffers
+            ops.kv_write(ws["layers"][i]["qkv"], self.cache[i], b_idx, pos, c.n_heads)
+        last = torch.tensor([r * S + n - 1 for r, n in enumerate(lens)], device=eng.device)
+        torch.index_select(ws["h"][c.n_layers], 0, last, out=self.h[0])
+        self._head(self.h[0])
+        self.lengths = lens
+        return self.logits
+
+    @torch.no_grad()
+    def step(self, tokens: torch.Tensor, active: list[bool] | None = None) -> torch.Tensor:
+        """Append ``tokens [B]`` (device int64) at each row's next position; returns the next-token logits ``[B, V]``.
+        Rows with ``active[r] = False`` do not advance: their cache is left to be overwritten and their logits are unused."""
+        for r in range(self.B):
+            if active is None or active[r]:
+                if self.lengths[r] >= self.S_max:
+                    raise ValueError(f"row {r} is full ({self.S_max} positions)")
+                self.lengths[r] += 1
+        self.meta.copy_(torch.tensor([self.lengths, [n - 1 for n in self.lengths]], dtype=torch.int32))
+        self.tokens.copy_(tokens)
+        if not self.eng.use_graph:
+            self._step_body()
+        else:
+            if self._graph is None:
+                self._capture()
+            self._graph.replay()
+        return self.logits
+
+    def _capture(self) -> None:
+        side = torch.cuda.Stream(self.eng.device)
+        side.wait_stream(torch.cuda.current_stream(self.eng.device))
+        with torch.cuda.stream(side):
+            self._step_body()        # warm-up: the same step the replay below recomputes
+        torch.cuda.current_stream(self.eng.device).wait_stream(side)
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            self._step_body()
+        self._graph = graph
+
+    def _head(self, h: torch.Tensor) -> None:
+        eng, c, bf = self.eng, self.eng.cfg, self.buf
+        ops.layernorm_fwd(h, eng.gf, eng.bf, bf["ln"], bf["m"], bf["r"], c.norm_eps)
+        ops.gemm(bf["ln"], eng.wte16, self.logits)
+
+    def _step_body(self) -> None:
+        eng, c, bf = self.eng, self.eng.cfg, self.buf
+        lengths, pos = self.meta[0], self.meta[1]
+        ops.embed_at(self.tokens, pos, eng.wte16, eng.wpe16, self.h[0])
+        scale = 1.0 / math.sqrt(c.d_head)
+        for i, w in enumerate(eng.layers):
+            h, h_next = self.h[i % 2], self.h[(i + 1) % 2]
+            ops.layernorm_fwd(h, w.g1, w.b1, bf["ln"], bf["m"], bf["r"], c.norm_eps)
+            ops.linear_fwd(bf["ln"], w.wqkv, w.bqkv, bf["qkv"])
+            if c.clip_qkv:
+                bf["qkv"].clamp_(-c.clip_qkv, c.clip_qkv)
+            if c.qk_ln:
+                qkv3 = bf["qkv"].view(-1, 3, c.d_model)
+                for j in range(2):
+                    bf["qk_pre"].copy_(qkv3[:, j])
+                    ops.layernorm_fwd(bf["qk_pre"], w.qk_g[j], w.qk_b[j], bf["qk_tmp"], bf["m"], bf["r"], c.norm_eps)
+                    qkv3[:, j].copy_(bf["qk_tmp"])
+            ops.kv_write(bf["qkv"], self.cache[i], self.b_idx, pos, c.n_heads, rope=eng.rope)
+            ops.decode_attention(bf["qkv"], self.cache[i], lengths, eng.alibi, scale, c.n_heads, bf["attn"], n_split=self.n_split)
+            ops.linear_fwd(bf["attn"], w.wo, w.bo, bf["hmid"], residual=h)
+            ops.layernorm_fwd(bf["hmid"], w.g2, w.b2, bf["ln"], bf["m"], bf["r"], c.norm_eps)
+            ops.linear_gelu_grad_fwd(bf["ln"], w.wup, w.bup, bf["z"], bf["u"])
+            ops.linear_fwd(bf["u"], w.wdown, w.bdown, h_next, residual=bf["hmid"])
+        self._head(self.h[c.n_layers % 2])

@@ -265,3 +265,45 @@ def rope_(qkv: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor, n_heads: int,
     transposed rotation (what the gradients of q and k need)."""
     ext().rope(qkv, cos, sin, int(n_heads), bool(inverse))
     return qkv
+
+
+# ---------------------------------------------------------------------------- KV-cached decoding
+def embed_at(ids: torch.Tensor, pos: torch.Tensor, wte: torch.Tensor, wpe: torch.Tensor | None, out: torch.Tensor) -> torch.Tensor:
+    """``out[t] = wte[ids[t]] (+ wpe[pos[t]])``: int64 ids, int32 explicit positions (``embed_fwd`` derives them as ``t % S``).
+    Out-of-range ids are clamped as in ``embed_fwd``."""
+    ext().embed_at(ids, pos, wte, wpe, out)
+    return out
+
+
+def decode_attention_splits(bh: int, s_max: int) -> int:
+    """The key-split count :func:`decode_attention` picks for ``bh`` (row, head) pairs over an ``s_max`` cache."""
+    return int(ext().decode_attention_splits(int(bh), int(s_max)))
+
+
+def decode_attention(q: torch.Tensor, kv: torch.Tensor, lengths: torch.Tensor, alibi_slopes: torch.Tensor | None, scale: float,
+                     n_heads: int, out: torch.Tensor, lse: torch.Tensor | None = None, n_split: int = 0) -> torch.Tensor:
+    """One query per row against a ragged KV cache (split-KV flash-decoding).
+
+    ``q``: bf16 rows ``[B, >= d]`` (the q third of the step's ``qkv [B, 3d]`` is ``qkv`` itself: only the first ``d`` columns
+    are read); ``kv``: bf16 ``[B, S_max, 2d]`` (k | v, head-major); ``lengths``: int32 ``[B]`` valid keys per row on the device,
+    the current token included; ``alibi_slopes``: optional fp32 ``[H]`` (adds ``slope_h * (key - (length - 1))``). Keys at or
+    beyond ``length`` are never read. ``out``: bf16 ``[B, d]``; ``lse``: optional fp32 ``[B, H]`` (natural log).
+    ``n_split`` = 0 picks :func:`decode_attention_splits`; it depends only on shapes, so a captured step stays valid."""
+    ext().decode_attention(q, kv, lengths, alibi_slopes, float(scale), int(n_heads), int(n_split), out, lse)
+    return out
+
+
+def kv_write(qkv: torch.Tensor, cache: torch.Tensor, b_idx: torch.Tensor, pos: torch.Tensor, n_heads: int,
+             rope: tuple[torch.Tensor, torch.Tensor] | None = None) -> None:
+    """``cache[b_idx[t], pos[t]] = k | v`` of ``qkv [T, 3d]`` row ``t`` (int32 coordinates). With ``rope`` = (cos, sin) the
+    row's q and k are first rotated in place at ``pos[t]``, bit-identical to :func:`rope_` at that position."""
+    cos, sin = rope if rope is not None else (None, None)
+    ext().kv_write(qkv, cache, b_idx, pos, cos, sin, int(n_heads))
+
+
+def argmax_rows(logits: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+    """int64 ``[R]`` index of the largest value of every bf16 row of ``logits [R, V]``; ties go to the lowest index."""
+    if out is None:
+        out = torch.empty(logits.shape[0], dtype=torch.int64, device=logits.device)
+    ext().argmax_rows(logits, out)
+    return out

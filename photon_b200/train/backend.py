@@ -16,11 +16,12 @@ Protocol
                               returns device scalars ``(loss_sum, n_tokens)``
 ``eval_stats(ids)``           ``{"loss_sum","n_tokens","n_correct"[, "unigram_loss_sum"]}``
 ``params_updated()``          hook after optimizer / parameter load (refresh shadows)
+``generate(prompts, max_new_tokens, eos_id, stop)``  batched greedy decoding (the engine: with a KV cache)
 """
 from __future__ import annotations
 
 import contextlib
-from typing import Any
+from typing import Any, Callable
 
 import torch
 import torch.nn.functional as F
@@ -131,6 +132,39 @@ class TorchBackend:
         """``[B,S] → [B,S,V]`` next-token logits (the in-context-learning evaluator's view of the model)."""
         with autocast_ctx(self.device, self.precision):
             return self.model(ids.to(self.device))
+
+    @torch.no_grad()
+    def generate(self, prompts: list[list[int]], max_new_tokens: int, eos_id: int | None = None,
+                 stop: Callable[[int, list[int]], bool] | None = None) -> list[list[int]]:
+        """Greedy continuation of every prompt by batched recompute (no cache); returns the new ids of each row.
+
+        Each step runs the unfinished rows' windows (the last ``max_seq_len`` ids) right-padded in one batch and takes every
+        row's argmax at its last valid position; causal attention keeps the padding out of the valid positions. A row ends
+        at ``eos_id`` (not included), when ``stop(row, new_ids)`` returns True, or after ``max_new_tokens``."""
+        msl = self.cfg.max_seq_len
+        ctx = [list(p) for p in prompts]
+        new: list[list[int]] = [[] for _ in prompts]
+        done = [False] * len(prompts)
+        for _ in range(max_new_tokens):
+            rows = [r for r in range(len(prompts)) if not done[r]]
+            if not rows:
+                break
+            wins = [ctx[r][-msl:] for r in rows]
+            ids = torch.zeros(len(rows), max(len(w) for w in wins), dtype=torch.long)
+            for j, w in enumerate(wins):
+                ids[j, : len(w)] = torch.tensor(w, dtype=torch.long)
+            logits = self.logits(ids)
+            last = torch.tensor([len(w) - 1 for w in wins], device=logits.device)
+            nxt = logits[torch.arange(len(rows), device=logits.device), last].float().argmax(-1).tolist()
+            for r, t in zip(rows, nxt):
+                if eos_id is not None and t == eos_id:
+                    done[r] = True
+                    continue
+                ctx[r].append(t)
+                new[r].append(t)
+                if stop is not None and stop(r, new[r]):
+                    done[r] = True
+        return new
 
     def params_updated(self) -> None:
         pass

@@ -430,7 +430,9 @@ class Trainer:
         vals = st.eval_metric_values
         self.log({f"metrics/{k}": v for k, v in vals.items()})
         if self.icl_suite is not None:   # llm-foundry's ICL evaluators + EvalGauntlet run as part of every trainer.eval()
-            icl = {k: v for k, v in self.icl_suite(st.backend.logits).items() if isinstance(v, (int, float))} if self.rank == 0 else {}
+            # generation tasks decode batched through the backend (on the engine: KV-cached, on its own kernels)
+            gen = st.backend.generate if st.backend.kind == "torch" or getattr(st.backend, "can_generate", False) else None
+            icl = {k: v for k, v in self.icl_suite(st.backend.logits, gen).items() if isinstance(v, (int, float))} if self.rank == 0 else {}
             self.last_icl_metrics = icl
             if self.world_size > 1 and dist.is_initialized():
                 # the suite runs on rank 0 only and can take minutes: the others wait HERE, on the host, instead of inside the next
